@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the clap procedural-generation hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Metric (BASELINE.json): CA cell-updates per second (GCUPS) for ca3d_run() -- core/ca3d.c:124-142 -- on a
 synthetic 2048^3 uint8 volume, 50 generations of ca_coral (BASELINE config 4; fits one GPU, so it is also the
@@ -25,6 +25,9 @@ N = 1 workload).  One "step" = one full run of all generations over the volume.
              cfg 1 (ca2d 256^2 x 5), cfg 2 (ca3d 128^3 x 10), cfg 3 (ca2d 16384^2 x 100; and once more on the diagonal
              engine, which is not the default), cfg 5 (terrain 8192^2),
              the 256^3 noise bake and the 8192^2 mesh, each with value / roofline / cpu_baseline / e2e / clocks.
+
+  --dump-outputs DIR  after the timed steps, the outputs of the last one as DIR/<name>.npy (see dump_outputs()), so that
+             two builds can be compared output for output: every input is generated from fixed seeds.
 
 Rank 0 prints exactly one JSON line.
 """
@@ -85,7 +88,61 @@ def parse():
                     help="repeat a short workload inside the timed region until it has lasted this long (clock samples)")
     ap.add_argument("--write-plane-hashes", action="store_true",
                     help="N = 1: write tests/golden/plane_hashes_<workload>.json (the fingerprints N > 1 runs are compared with)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MiB in all: a fixed sample of a larger output)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
+
+
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed in its last step
+# ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 0xD0
+
+
+def dump_index(n, cap):
+    """The flat indices --dump-outputs keeps of an output of n elements: all of them when n <= cap, else the sorted
+    distinct values among cap draws of numpy.random.default_rng(DUMP_SEED) -- the same in every run."""
+    import numpy as np
+    if n <= cap:
+        return np.arange(n)
+    return np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, cap))
+
+
+def u64_halves(h):
+    """uint64 fingerprints as [n, 2] int64 (high, low 32 bits): exact once written as float64"""
+    import numpy as np
+    return np.stack([h >> np.uint64(32), h & np.uint64(0xFFFFFFFF)], 1).astype(np.int64)
+
+
+def dump_outputs(directory, arrays):
+    """Write each output (name -> torch tensor on any device, or numpy array) as <directory>/<name>.npy: integers of up
+    to 16 bits and float32 as float32, wider integers as float64, all exact.  An output with more elements than its
+    share of DUMP_BYTES allows is written flat, reduced to the elements dump_index() picks."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    cap = DUMP_BYTES // 8 // len(arrays)
+    total = 0
+    for name, a in arrays.items():
+        t = torch.as_tensor(a)
+        shape = tuple(t.shape)
+        t = t.reshape(-1)
+        idx = dump_index(t.numel(), cap)
+        if len(idx) < t.numel():
+            t, shape = t[torch.from_numpy(idx).to(t.device)], (len(idx),)
+        v = t.cpu().numpy().reshape(shape)
+        v = v.astype(np.float32 if v.dtype == np.float32 or v.dtype.itemsize <= 2 else np.float64)
+        np.save(os.path.join(directory, name + ".npy"), v)
+        total += v.nbytes
+    assert total <= DUMP_BYTES, total
+    print(f"bench: {len(arrays)} outputs of the last timed step ({total / 2 ** 20:.1f} MiB) in {directory}", file=sys.stderr)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -321,6 +378,12 @@ def run_ca3d(args, torch, clap_b200, dev, local, workload, headline=True):
     wall = time.perf_counter() - t_wall0
     clocks = sampler.stop()
     hashes = hash_planes(grid.device_ptr(), d0 * d1, d2)
+    if args.dump_outputs:
+        # the volume is too large to keep whole: a sample of its cells, and every plane through its fingerprint
+        final = torch.empty_like(seed_dev)
+        grid.download(final.data_ptr())
+        dump_outputs(args.dump_outputs, {"volume": final, "population": np.array([pop]), "plane_hashes": u64_halves(hashes)})
+        del final
 
     ms_per_step = tot_ms / nsteps
     value = updates / (ms_per_step * 1e-3) / 1e9
@@ -555,6 +618,12 @@ def run_ca2d(args, torch, clap_b200, dev, local, workload):
     torch.cuda.synchronize()
     clocks = sampler.stop()
     pop = grid.count()
+    if args.dump_outputs:
+        from clap_b200.ca import hash_planes
+        final = torch.empty_like(seed_dev)
+        grid.download(final.data_ptr())
+        dump_outputs(args.dump_outputs, {"grid": final, "row_hashes": u64_halves(hash_planes(grid.device_ptr(), side, side))})
+        del final
     # BASELINE config 3 at full size was run ONCE through the unmodified reference (tests/golden/make_golden_cfg3.py):
     # the population of the final grid must be the reference's
     ref_pop = None
@@ -685,6 +754,9 @@ def run_fields(args, torch, clap_b200, dev, local, workload):
                                                                 1.0, 4, byref(a), byref(b)))
             return a.value + b.value, b.value, 2 if os.environ.get("CLAPCA_TERRAIN_DIRECT") else 3
 
+        def outputs():
+            return {"heightmap": d_map, "map0": d_map0}
+
         host_out = torch.empty(units, dtype=torch.float32, pin_memory=True)
 
         def e2e_step():
@@ -720,6 +792,10 @@ def run_fields(args, torch, clap_b200, dev, local, workload):
                                                            c_void_p(d_tx.data_ptr()), c_void_p(d_idx.data_ptr()), byref(a)))
             return a.value, a.value, 2
 
+        def outputs():
+            # the index buffer holds C unsigned shorts in an int16 tensor: dumped as their unsigned values
+            return {"vertices": d_vx, "normals": d_norm, "uv": d_tx, "indices": d_idx.to(torch.int32) & 0xFFFF}
+
         host_map = torch.empty(units, dtype=torch.float32, pin_memory=True)
         host_map.copy_(d_map)
         h_vx = torch.empty(units * 3, dtype=torch.float32, pin_memory=True)
@@ -751,6 +827,9 @@ def run_fields(args, torch, clap_b200, dev, local, workload):
                                                          byref(a)))
             return a.value, a.value, 2
 
+        def outputs():
+            return {"rgba": d_out.view(torch.uint8)}
+
         host_out = torch.empty(units, dtype=torch.int32, pin_memory=True)
 
         def e2e_step():
@@ -772,6 +851,8 @@ def run_fields(args, torch, clap_b200, dev, local, workload):
         tot_ms += t; ker_ms += k; launches += n
         nsteps += 1
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs())
     ms_per_step, kernel_ms = tot_ms / nsteps, ker_ms / nsteps
     if "hashes_per_voxel" in extra:
         extra["achieved_ghash_per_s"] = units * extra["hashes_per_voxel"] / (kernel_ms * 1e-3) / 1e9
@@ -887,6 +968,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if world > 1 and args.workload in WORKLOADS and args.dump_outputs:
+        raise SystemExit("--dump-outputs: a volume sharded over several GPUs is not written; run it on one GPU")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: there is no CPU fallback for the product path")
     torch.cuda.set_device(local)
@@ -917,7 +1000,7 @@ def main():
             sec = {}
             sargs = argparse.Namespace(**vars(args))
             sargs.steps, sargs.warmup, sargs.min_seconds, sargs.cpu_seconds = 3, 3, 1.5, 3.0
-            sargs.write_plane_hashes = False
+            sargs.write_plane_hashes, sargs.dump_outputs = False, None
             t0 = time.perf_counter()
             for name in SECONDARY:
                 try:

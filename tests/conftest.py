@@ -23,16 +23,6 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def reference():
-    """oracle/_ref/libclapref.so = the unmodified reference sources; skip when it was not built."""
-    import oracle_lib
-    ref = oracle_lib.ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/libclapref.so not built (needs /root/reference)")
-    return ref
-
-
-@pytest.fixture(scope="session")
 def gpu():
     """Bind the product library to cuda:0; fails (does not skip) when the CUDA path is unusable."""
     import clap_b200

@@ -43,7 +43,7 @@ def test_host_shim_exports_reference_entry_points():
             assert hasattr(lib, n), f"{n} ({header}) missing from libclapca_host.so"
 
 
-def test_rule_struct_layout_matches_reference():
+def test_rule_struct_layout_matches_reference(tmp_path):
     """struct cell_automaton is 32 bytes with the members at the reference's offsets (core/ca-common.h)."""
     src = r'''
     #include <stdio.h>
@@ -57,7 +57,7 @@ def test_rule_struct_layout_matches_reference():
                offsetof(struct cell_automaton, neigh_2d), offsetof(struct xyzarray, arr));
         return 0;
     }'''
-    exe = "/tmp/clapca_layout_test"
+    exe = str(tmp_path / "clapca_layout_test")
     subprocess.run(["gcc", "-std=gnu11", "-x", "c", "-", "-I", os.path.join(ROOT, "include", "clap"), "-o", exe],
                    input=src.encode(), check=True)
     out = subprocess.run([exe], capture_output=True, check=True).stdout.split()

@@ -90,11 +90,11 @@ int main(void)
 '''
 
 
-def test_reference_style_c_program(oracle):
+def test_reference_style_c_program(oracle, tmp_path):
     lib_dir = os.path.join(ROOT, "clap_b200", "lib")
     if not all(os.path.exists(os.path.join(lib_dir, n)) for n in ("libclapca_cuda.so", "libclapca_host.so")):
         subprocess.run(["make", "-C", os.path.join(ROOT, "clap_b200", "csrc"), "-j8"], check=True, capture_output=True)
-    exe = "/tmp/clapca_shim_test"
+    exe = str(tmp_path / "clapca_shim_test")
     lib = os.path.join(ROOT, "clap_b200", "lib")
     subprocess.run(["gcc", "-std=gnu11", "-O1", "-x", "c", "-", "-I", os.path.join(ROOT, "include", "clap"),
                     "-L", lib, "-lclapca_host", "-lclapca_cuda", f"-Wl,-rpath,{lib}", "-o", exe],
