@@ -69,6 +69,16 @@ def test_ca3d_wide_rows_and_words_per_lane(emu_bin):
     _run(exe, 2048, 2, 2, 2, 7, 3, 2, 0, 9, 4)
 
 
+@pytest.mark.parametrize("nca,planes,wpl", [(nca, planes, wpl) for nca in range(11) for planes in (3, 4, 8)
+                                             for wpl in (1, 2, 4) if not (planes == 3 and nca in (2, 4))])
+def test_ca3d_every_rule_planes_and_words_per_lane(emu_bin, nca, planes, wpl):
+    """The full (rule, state planes, words per lane) matrix the library instantiates, on ragged rows of each width
+    class (pyroclastic and builder, nr_states 10, need at least 4 planes)."""
+    width = {1: 1000, 2: 2047, 4: 3999}[wpl]
+    seedkind = {3: 0, 4: 1, 8: 2}[planes]      # values 0..5, dense 0..15, the ca3d_make seed with its 255s
+    _run(os.path.join(emu_bin, "emu_ca3d"), width, 3, 3, 2, nca, planes, wpl, seedkind, nca * 9 + planes + wpl, 5)
+
+
 def test_ca3d_many_generations_few_and_many_workers(emu_bin):
     exe = os.path.join(emu_bin, "emu_ca3d")
     _run(exe, 24, 12, 10, 12, 10, 8, 1, 1, 3, 12)
@@ -268,6 +278,8 @@ def test_ca2d_rule_instantiations_agree(emu_bin, args):
     (7, 2050, 3, 0xc, 0x180, 4, 1, 1, 3, 1, 3, 0, 4, 1, 3),           # a single CTA runs every generation in turn
     (5, 4200, 2, 0x1e0, 0x1f0, 1, 1, 1, 1, 4, 2, 0, 5, 2, 2),
     (9, 1025, 5, 0x1fe, 0x0, 3, 1, 1, 3, 1, 2, 1, 9, 3, 2),           # one cell beyond a warp's span
+    (2, 32800, 2, 0x1e0, 0x1f0, 1, 1, 1, 1, 4, 16, 0, 10, 2, 2),      # 16 warps x 4 words (the widest row variant)
+    (3, 16400, 2, 0x1e, 0xff, 20, 0, 1, 8, 2, 16, 1, 11, 2, 2),       # 8 planes: 16 warps x 2 words
 ])
 def test_ca2d_bitplane_rows_across_warps(emu_bin, args):
     _run(os.path.join(emu_bin, "emu_ca2d"), *args)
