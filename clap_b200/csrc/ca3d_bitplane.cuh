@@ -66,6 +66,8 @@ struct Bp3Params {
     int nsweeps;            /* number of work items */
     int flag_rows;          /* progress counters are raised every flag_rows rows (and at segment ends) */
     int prefetch_rows;      /* > 0: prefetch.L2 the own record this many rows ahead (HBM -> L2 latency) */
+    int rowloop_generic;    /* != 0: every row takes the general row step, none the interior one (CLAPCA_ROWLOOP=generic:
+                               A/B runs and parity checks of the two row loops) */
     unsigned *ticket;       /* next sweep to claim */
     int *err;               /* != 0: watchdog fired, everybody bails out */
     unsigned long long *diag;   /* optional: cycles [0] waiting on gpu-scope counters, [1] service warps busy, [2] in work items,
@@ -286,22 +288,35 @@ struct Sweep3 {
                                                        uniform-datapath instruction in a loop that is bound by issue) */
         PubSlot *slot;                              /* publisher mode: this worker's mailbox (else nullptr) */
         const int *sprod;                           /* tile mode: lanes 0..2 = shared-memory row counter of producer dn / up / own */
-        int *sown;                                  /* tile mode: own shared-memory row counter (else nullptr) */
+        int *sown;                                  /* tile mode: own shared-memory row counter */
         int have_s;                                 /* min over the rows the tile-mates have published through sprod */
         const int *flagp;                           /* the gpu-scope producer counter this lane polls (lanes 0..2) */
         bool flag_sys;                              /* ... is written by another GPU: poll at system scope */
         int have;                                   /* min over the producers' published row counts */
+        int have_min;                               /* min(have_s, have): the fast path of a dependency check is ONE compare */
         int next_raise;                             /* next row count at which the own counter is raised */
-        long long waited_flag, waited_team;         /* diagnostics: cycles spent in the slow paths */
     };
 
-    /* false = watchdog fired / abort requested */
+    /* rows < need of every producer are complete and visible.  false = watchdog fired / abort requested */
+    template <bool TILE>
     CA_MDEV bool wait_rows(const Bp3Params &p, St &st, int need)
     {
-        if (st.have_s < need && !wait_tile(p, st, need))
-            return false;
-        if (st.have >= need)
+        if (st.have_min >= need)
             return true;
+        if (TILE && st.have_s < need && !wait_tile(p, st, need))
+            return false;
+        if (st.have < need && !wait_flags(p, st, need))
+            return false;
+        st.have_min = (TILE && st.have_s < st.have) ? st.have_s : st.have;
+        return true;
+    }
+
+    /*
+     * Producers outside the tile (or every producer, one warp per sweep): lanes 0..2 poll the gpu- / system-scope
+     * counter of producer dn / up / own with ld.acquire, redux.min gives the row count all of them have reached.
+     */
+    CA_MDEV bool wait_flags(const Bp3Params &p, St &st, int need)
+    {
         long long t0 = 0;
         for (unsigned spins = 0;; spins++) {
             int v = 0x7fffffff;
@@ -323,7 +338,8 @@ struct Sweep3 {
                 }
             }
         }
-        if (t0) st.waited_flag += dp_clock() - t0;
+        if (t0 && p.diag && dp_lane() == 0)
+            dp_atomic_add64(p.diag + 0, (unsigned long long)(dp_clock() - t0));
         dp_syncwarp();          /* the polling lanes acquired; the warp barrier extends it to every lane */
         return true;
     }
@@ -356,7 +372,8 @@ struct Sweep3 {
             }
             dp_team_pause();
         }
-        if (t0) st.waited_team += dp_clock() - t0;
+        if (t0 && p.diag && dp_lane() == 0)
+            dp_atomic_add64(p.diag + 3, (unsigned long long)(dp_clock() - t0));
         dp_fence_cta();
         return true;
     }
@@ -411,8 +428,10 @@ struct Sweep3 {
      * One row step.  M = (y - y0) % 3 selects the register slots: rows y-1 / y / y+1 of the side planes
      * sit in slots (M+2)%3 / M / (M+1)%3, own state rows y / y+1 in slots M / (M+1)%3; row y+2 is
      * prefetched into slot (M+2)%3 once row y-1 has been consumed.
+     * TILE: tile mode (shared-memory row counter after every row) or one warp per sweep -- fixed per call site.
+     * INT: an interior row, y + 2 <= y1, y + 2 < H and y + prefetch_rows < H (run_rows): no edge test, no zero arm.
      */
-    template <int M>
+    template <int M, bool TILE, bool INT>
     CA_MDEV bool step(const Bp3Params &p, St &st, int y, int y1, int *myprog)
     {
         constexpr int A = (M + 2) % 3, B = M, C = (M + 1) % 3;
@@ -446,14 +465,19 @@ struct Sweep3 {
         }
 
         /* ---- prefetch row y+2 while the rule / scan / update below run ---- */
-        if (st.pf) {
-            if (y + p.prefetch_rows < H)
+        if (st.pf) {                /* a lane test, not a branch: the prefetch and the add are predicated */
+            if (INT || y + p.prefetch_rows < H)
                 dp_prefetch_l2(st.pf);
             st.pf += RECW;
         }
         if (y + 2 <= y1) {          /* row y1 is still needed (as "row y+1" of the last step), y1+1 is not */
-            if (y + 2 < H) {
-                if (!wait_rows(p, st, y + 3 < H ? y + 3 : H))
+            /*
+             * Always true on an interior row, where it is the one test left: without this branch around the wait
+             * and the loads ptxas schedules the interior step with ~20 more instructions per row (it
+             * rematerialises the valid-cell mask and the counter address; tools/sass_hist.py).
+             */
+            if (INT || y + 2 < H) {
+                if (!wait_rows<TILE>(p, st, (INT || y + 3 < H) ? y + 3 : H))
                     return false;
                 load_own_h<2>(st, st.ho);
                 load_own_s<2>(st, st.so[A]);
@@ -526,26 +550,25 @@ struct Sweep3 {
         for (int q = 0; q < P; q++)
             LaneVec<WPL>::st(st.rec + (2 + q) * RWP, st.so[B][q]);
         st.rec += RECW;
-        if (st.sown) {
+        if (TILE) {
             /*
-             * Tile mode: warp barrier (orders every lane's row stores before lane 0), CTA-scope release, row
-             * counter in shared memory -- after EVERY row.  The service warp carries it to gpu / system scope.
+             * Tile mode: warp barrier (orders every lane's row stores before lane 0), CTA-scope release by lane 0,
+             * row counter in shared memory -- after EVERY row.  The service warp carries it to gpu / system scope.
+             * Lane 0's fence and store are predicated, not branched around: the warp never diverges, so the next
+             * step's shuffles and votes need no convergence check.
              */
             dp_syncwarp();
-            if (lane == 0) {
-                dp_fence_cta();
-                dp_st_volatile(st.sown, y + 1);
-            }
+            dp_release_cta_if(lane == 0, st.sown, y + 1);
             return true;
         }
         /*
          * One warp per sweep: warp barrier, then ONE release store of the counter (MEMBAR.GPU + store), or the
-         * publisher's mailbox.  Raised every flag_rows rows.
+         * publisher's mailbox.  Raised every flag_rows rows, and after the item's last row (never an interior row).
          */
         const bool at_mark = (y + 1 == st.next_raise);
         if (at_mark)
             st.next_raise += p.flag_rows;
-        if (at_mark || y + 1 == y1) {
+        if (at_mark || (!INT && y + 1 == y1)) {
             dp_syncwarp();
             if (lane == 0) {
                 if (st.slot) {
@@ -559,7 +582,8 @@ struct Sweep3 {
         return true;
     }
 
-    /* one work item: rows [y0, y1) of plane z at generation g.  false = aborted */
+    /* one work item: rows [y0, y1) of plane z at generation g; TILE: tw is the tile's wiring, else nullptr.  false = aborted */
+    template <bool TILE>
     CA_MDEV bool run_rows(const Bp3Params &p, int z, int g, int y0, int y1, PubSlot *slot, const TileWire *tw)
     {
         const int lane = dp_lane();
@@ -592,10 +616,13 @@ struct Sweep3 {
             st.sprod = lane == 0 ? sdn : (lane == 1 ? sup : (lane == 2 ? sow : nullptr));
             st.have_s = (sdn || sup || sow) ? 0 : 0x7fffffff;
         }
-        st.sown = tw ? tw->done : nullptr;
+        st.have_min = st.have_s < st.have ? st.have_s : st.have;
+        st.sown = TILE ? tw->done : nullptr;
         st.next_raise = (y0 / p.flag_rows + 1) * p.flag_rows;
-        st.waited_flag = st.waited_team = 0;
-        const long long t_item = dp_clock();
+        /* diagnostics go straight to the counters (the item's time as - start + end): no clock lives in a register
+           across the row loop, whose register budget is exhausted */
+        if (p.diag && lane == 0)
+            dp_atomic_add64(p.diag + 2, 0ull - (unsigned long long)dp_clock());
 #pragma unroll
         for (int j = 0; j < WPL; j++) st.vmask[j] = bp_valid_mask(lane * WPL + j, p.W);
 
@@ -631,7 +658,7 @@ struct Sweep3 {
             dp_fence_cta();
             dp_st_volatile(&slot->pub, y0);
         }
-        if (!wait_rows(p, st, y0 + 2 < H ? y0 + 2 : H))
+        if (!wait_rows<TILE>(p, st, y0 + 2 < H ? y0 + 2 : H))
             return false;
 
         /* ---- fill the windows: pair sums of rows y0-1 (slot 2) and y0 (slot 0); row y0+1 waits in hd / hu ---- */
@@ -662,18 +689,25 @@ struct Sweep3 {
 #pragma unroll
         for (int j = 0; j < WPL; j++) st.tt[1][0][j] = st.tt[1][1][j] = st.tt[1][2][j] = 0u;
 
+        /*
+         * Rows [y0, yi) are interior: every edge test of the general step has a result known here, so they take
+         * the step without them.  The rest (at most two of the interior rows, then the last rows of the item or
+         * of the plane) take the general step; the slots continue at M = 0 because yi - y0 rows is rounded to 3.
+         */
+        int yi = y1 - 1;                                /* y + 2 <= y1 */
+        if (yi > H - 2) yi = H - 2;                     /* y + 2 < H: row y + 2 exists, the wait is for y + 3 <= H rows */
+        if (yi > H - p.prefetch_rows) yi = H - p.prefetch_rows;     /* the prefetched line is inside the plane */
+        if (p.rowloop_generic) yi = y0;
         int y = y0;
-        for (; y + 3 <= y1; y += 3) {
-            if (!step<0>(p, st, y, y1, myprog)) return false;
-            if (!step<1>(p, st, y + 1, y1, myprog)) return false;
-            if (!step<2>(p, st, y + 2, y1, myprog)) return false;
+        for (; y + 3 <= yi; y += 3) {
+            if (!step<0, TILE, true>(p, st, y, y1, myprog)) return false;
+            if (!step<1, TILE, true>(p, st, y + 1, y1, myprog)) return false;
+            if (!step<2, TILE, true>(p, st, y + 2, y1, myprog)) return false;
         }
-        if (y < y1) {
-            if (!step<0>(p, st, y, y1, myprog)) return false;
-            y++;
-        }
-        if (y < y1) {
-            if (!step<1>(p, st, y, y1, myprog)) return false;
+        for (; y < y1; y += 3) {
+            if (!step<0, TILE, false>(p, st, y, y1, myprog)) return false;
+            if (y + 1 < y1 && !step<1, TILE, false>(p, st, y + 1, y1, myprog)) return false;
+            if (y + 2 < y1 && !step<2, TILE, false>(p, st, y + 2, y1, myprog)) return false;
         }
         /* publisher mode: the mailbox is reused by the next item only once the last rows are out */
         if (slot) {
@@ -682,11 +716,8 @@ struct Sweep3 {
                     dp_nanosleep(20);
             dp_syncwarp();
         }
-        if (p.diag && lane == 0) {
-            dp_atomic_add64(p.diag + 0, (unsigned long long)st.waited_flag);
-            dp_atomic_add64(p.diag + 2, (unsigned long long)(dp_clock() - t_item));
-            dp_atomic_add64(p.diag + 3, (unsigned long long)st.waited_team);
-        }
+        if (p.diag && lane == 0)
+            dp_atomic_add64(p.diag + 2, (unsigned long long)dp_clock());
         return true;
     }
 
@@ -854,7 +885,7 @@ struct Sweep3 {
             if (g >= p.G)
                 return unpack_plane(p, z);
         }
-        return run_rows(p, z, g, y0, y1, slot, nullptr);
+        return run_rows<false>(p, z, g, y0, y1, slot, nullptr);
     }
 
     /* the worker loop: claim items in dependency order until the list is exhausted */
@@ -1166,10 +1197,14 @@ struct Sweep3 {
             const int4 it = p.order[t];
             const int nz = it.z & 0xff, ng = (it.z >> 8) & 0xff;
             if (p.layout_items && (it.y < 0 || it.y >= p.G)) {
-                if (w < nz)
-                    run_item(p, it.x + w, it.y, 0, p.H, nullptr);
-                else if (w == T && it.y < 0)
+                if (w < nz) {
+                    if (it.y < 0)
+                        pack_plane(p, it.x + w);
+                    else
+                        unpack_plane(p, it.x + w);
+                } else if (w == T && it.y < 0) {
                     seed_push(p, it.x, ts, phase);  /* a packed z-block edge is the neighbour's "old plane above" of generation 0 */
+                }
             } else if (w < nz * ng) {
                 const int i = w % nz, j = w / nz;
                 TileWire tw;
@@ -1177,7 +1212,7 @@ struct Sweep3 {
                 tw.up = (j > 0 && i + 1 < nz) ? sm + (w - nz + 1) : nullptr;
                 tw.own = j > 0 ? sm + (w - nz) : nullptr;
                 tw.done = sm + w;
-                run_rows(p, it.x + i, it.y + j, 0, p.H, nullptr, &tw);
+                run_rows<true>(p, it.x + i, it.y + j, 0, p.H, nullptr, &tw);
             } else if (w == T) {
                 service_loop(p, it.x, it.y, nz, ng, ts, phase);
             }

@@ -558,6 +558,8 @@ void clapca::api::sweep_knobs(Bp3Params &p, int team, bool single_gpu)
     if (const char *e = getenv("CLAPCA_CTAS_PER_SM")) p.max_ctas_per_sm = std::max(0, atoi(e));
     if (const char *e = getenv("CLAPCA_MAX_CTAS")) p.max_ctas = std::max(0, atoi(e));
     if (const char *e = getenv("CLAPCA_PUB_WORKERS")) p.pub_workers = std::max(0, atoi(e));
+    /* CLAPCA_ROWLOOP=generic: every row takes the general row step (same volumes; A/B of the interior row loop) */
+    if (const char *e = getenv("CLAPCA_ROWLOOP")) p.rowloop_generic = strcmp(e, "generic") == 0;
     p.team = team;
     /*
      * Halo rows: batched ld / st of the service warp by default.  The TMA variant (1-D bulk copies record -> shared

@@ -160,6 +160,16 @@ CA_DEV uint32_t dp_funnel_l_clamp(uint32_t lo, uint32_t hi, uint32_t s) { return
  * the copy itself runs in the async proxy, off the issuing warp.  Addresses and sizes are multiples of 16 bytes.
  */
 CA_DEV uint32_t dp_smem_addr(const void *p)       { return (uint32_t)__cvta_generic_to_shared(p); }
+/*
+ * CTA-scope release of a shared-memory counter by the lanes with `pub`: fence.acq_rel.cta, then the volatile store, with
+ * no branch, so the warp never diverges.  The whole warp executes the fence (ptxas branches around a predicated MEMBAR;
+ * it is one MEMBAR per warp either way) and only the `pub` lanes store.  p points into shared memory.
+ */
+CA_DEV void dp_release_cta_if(bool pub, int *p, int v)
+{
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tfence.acq_rel.cta;\n\t@q st.volatile.shared.s32 [%0], %1;\n\t}"
+                 :: "r"(dp_smem_addr(p)), "r"(v), "r"((uint32_t)pub) : "memory");
+}
 CA_DEV void dp_mbar_init(unsigned long long *bar, int arrivals)
 {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(dp_smem_addr(bar)), "r"(arrivals) : "memory");
@@ -346,6 +356,14 @@ CA_DEV uint32_t dp_funnel_r(uint32_t lo, uint32_t hi, int s)
 CA_DEV uint32_t dp_funnel_l_clamp(uint32_t lo, uint32_t hi, uint32_t s)
 {
     return s >= 32 ? lo : (s ? (hi << s) | (lo >> (32 - s)) : hi);
+}
+
+CA_DEV void dp_release_cta_if(bool pub, int *p, int v)
+{
+    if (pub) {
+        __atomic_thread_fence(__ATOMIC_SEQ_CST);
+        __atomic_store_n(p, v, __ATOMIC_RELEASE);
+    }
 }
 
 /*
